@@ -14,6 +14,10 @@ add, 24.375 B/row algorithmic) from its own CUDA-event time inside the timed reg
 
 `--impl reference` times the CPU restatement of the reference (oracle/, arrow-rs cannot be
 built here: no Rust toolchain) on the host cores, row-partitioned over all of them.
+
+`--dump-outputs DIR` writes what the last timed step returned (filter, take and add outputs with
+their validity, the sum) as .npy files of finite float64 / float32 values, so that two builds can
+be compared output for output on the same seeded inputs.
 """
 import argparse
 import ctypes as C
@@ -21,6 +25,8 @@ import json
 import os
 import subprocess
 import sys
+
+sys.dont_write_bytecode = True  # the benchmark may run from a read-only tree: no __pycache__ next to the sources
 
 # The contract is ONE JSON line on stdout. Libraries loaded later (NCCL prints "NCCL version ..." when NCCL_DEBUG is set)
 # write to file descriptor 1 directly, so the real stdout is set aside and fd 1 is pointed at stderr for everything else.
@@ -293,6 +299,57 @@ def gpu_checksums(ctx, abi, wl):
     return {"filter_rows": int(wl.out_filter.len), "filter_nulls": nulls(wl.out_filter), "filter_values_wsum": wsum(wl.out_filter),
             "take_nulls": nulls(wl.out_take), "take_values_wsum": wsum(wl.out_take), "add_nulls": nulls(wl.out_add),
             "add_bits_wsum": wsum(wl.out_add), "sum_valid_rows": int(cnt), "sum_bits": int(bits), "valid_rows": int(cnt)}
+
+
+# --dump-outputs: an output longer than DUMP_ROWS is sampled as DUMP_ROWS // DUMP_BLOCK blocks of DUMP_BLOCK rows, so the
+# three step outputs take 3 x 2^20 rows x (8 B values + 4 B validity) = 36 MiB at any table size (a dump stays under 64 MiB).
+DUMP_ROWS, DUMP_BLOCK, DUMP_SEED = 1 << 20, 1 << 12, 47
+
+
+def dump_rows(length):
+    """Rows of a `length`-row output that --dump-outputs writes: all of them up to DUMP_ROWS, else whole DUMP_BLOCK-row
+    blocks at seeded random offsets (the same rows on every run; block starts are multiples of 8, so every block's
+    validity is whole bitmap bytes)."""
+    if length <= DUMP_ROWS:
+        return np.arange(length)
+    blocks = np.random.default_rng(DUMP_SEED).choice(length // DUMP_BLOCK, DUMP_ROWS // DUMP_BLOCK, replace=False)
+    return (np.sort(blocks)[:, None] * DUMP_BLOCK + np.arange(DUMP_BLOCK)).ravel()
+
+
+def dump_output(ctx, out, dtype, out_dir, name):
+    """One step output (8-byte values, validity at bit offset 0), rows dump_rows(out.len): <name>.npy = the values as
+    float64, 0 in null slots (their contents are unspecified, so builds may differ there); <name>_valid.npy = the
+    validity as float32 1 / 0."""
+    n = int(out.len)
+    rows = dump_rows(n)
+    runs = [(0, n)] if len(rows) == n else [(int(s), DUMP_BLOCK) for s in rows[::DUMP_BLOCK]]
+    vals, valid = [], []
+    for start, count in runs:
+        vals.append(ctx.d2h(out.values + start * 8, count * 8, dtype))
+        if out.has_validity:
+            bits = ctx.d2h(out.validity + start // 8, (count + 7) // 8)
+            valid.append(np.unpackbits(bits, bitorder="little")[:count].astype(bool))
+    x = np.concatenate(vals).astype(np.float64)
+    v = np.concatenate(valid) if out.has_validity else np.ones(len(x), dtype=bool)
+    x[~v] = 0.0
+    np.save(os.path.join(out_dir, name + ".npy"), x)
+    np.save(os.path.join(out_dir, name + "_valid.npy"), v.astype(np.float32))
+
+
+def dump_outputs(ctx, wl, sum_bits, sum_valid, out_dir):
+    """--dump-outputs: what the last timed step returned to its caller (rank 0's shard when --gpus > 1), as .npy files:
+    filter / take (Int64 values) and add (Float64) by dump_output; sum = the all-reduced Int64 sum as float64 (0 when no
+    taken row is valid: arrow's None, told apart by the last count); counts = [filter rows, filter nulls, take rows,
+    take nulls, add rows, add nulls, valid rows of the sum], whole-output figures. Every value written is finite."""
+    os.makedirs(out_dir, exist_ok=True)
+    outs = (("filter", wl.out_filter, np.int64), ("take", wl.out_take, np.int64), ("add", wl.out_add, np.float64))
+    for name, out, dtype in outs:
+        dump_output(ctx, out, dtype, out_dir, name)
+    total = float(np.array([sum_bits], dtype=np.uint64).view(np.int64)[0]) if sum_valid else 0.0
+    np.save(os.path.join(out_dir, "sum.npy"), np.array([total]))
+    counts = [x for _, o, _ in outs for x in (o.len, o.null_count if o.has_validity else 0)] + [sum_valid]
+    np.save(os.path.join(out_dir, "counts.npy"), np.array(counts, dtype=np.float64))
+    print(f"bench.py: last step's outputs written to {out_dir}", file=sys.stderr)
 
 
 ALLREDUCE_WALL = [0.0, 0]  # host seconds spent inside the final-reduce call (includes waiting for the slowest rank), calls
@@ -625,6 +682,8 @@ def run_gpu(args):
         if cnt.value:
             kstats[name] = {"ms_per_step": tot.value / args.steps, "launches_per_step": cnt.value / args.steps,
                             "share_of_step": tot.value / ms.value}
+    if args.dump_outputs and rank == 0:  # here: the e2e arm and the oracle check below run the step again
+        dump_outputs(ctx, wl, total_bits, total_cnt, args.dump_outputs)
 
     # ---- e2e: host buffers, copies inside the timed region --------------------------------
     e2e = None
@@ -1034,7 +1093,12 @@ def main():
     ap.add_argument("--cpu-steps", type=int, default=5, help="timed CPU steps of the cpu_baseline leg of the GPU arm")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config sub-results (configs #2-#5)")
     ap.add_argument("--cpu-threads", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as .npy files to DIR (GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; the reference arm keeps its outputs inside oracle/refbench.cpp")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -74,3 +76,63 @@ def test_refbench_checksums_match_single_call_oracle():
     assert c["add_nulls"] == s.null_count and c["add_bits_wsum"] == wsum(s.values[: s.length])
     total = orc.sum(t)
     assert c["sum_bits"] == (int(total) & 0xFFFFFFFFFFFFFFFF) and c["valid_rows"] == t.length - t.null_count
+
+
+@pytest.mark.parametrize("args, message", [(("--steps", "0"), "--steps must be at least 1"),
+                                           (("--impl", "reference", "--dump-outputs", "out"), "--dump-outputs writes the GPU arm")])
+def test_bench_rejects_bad_arguments(args, message):
+    r = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), *args], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and message in r.stderr and not r.stdout
+
+
+def test_dump_rows_is_a_fixed_sample():
+    sys.path.insert(0, REPO)
+    import numpy as np
+    import bench
+    assert np.array_equal(bench.dump_rows(1000), np.arange(1000))
+    rows = bench.dump_rows(10 ** 9)
+    assert len(rows) == bench.DUMP_ROWS and np.array_equal(rows, bench.dump_rows(10 ** 9))
+    assert np.all(np.diff(rows) > 0) and rows[-1] < 10 ** 9 and np.all(rows[:: bench.DUMP_BLOCK] % 8 == 0)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_steps_outputs(tmp_path):
+    """--dump-outputs writes the last timed step's filter / take / add outputs (values and validity) and sum, all finite and
+    equal to the oracle's on the same seeded table: at 3e6 rows the add output (3e6 rows) is a sample, the filter and take
+    outputs are whole."""
+    sys.path.insert(0, REPO)
+    sys.path.insert(0, os.path.join(REPO, "arrow-rs_b200"))
+    sys.path.insert(0, os.path.join(REPO, "tests"))
+    import numpy as np
+    import bench
+    from acu import _abi as abi
+    from acu import HostArray, BOOL
+    from oracle import Oracle
+    n, out = 3_000_000, tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--rows", str(n), "--steps", "2", "--warmup", "1", "--no-e2e",
+                        "--no-cpu", "--no-configs", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][0])
+    assert line["steps"] == 2
+    got = {f[:-4]: np.load(out / f) for f in os.listdir(out)}
+    assert sorted(got) == ["add", "add_valid", "counts", "filter", "filter_valid", "sum", "take", "take_valid"]
+    assert all(v.dtype == (np.float32 if k.endswith("_valid") else np.float64) for k, v in got.items())
+    assert all(np.isfinite(v).all() for v in got.values()) and sum(v.nbytes for v in got.values()) <= 64 << 20
+    orc = Oracle()
+    col = HostArray(abi.I64, orc.generate_values(0, 42, 0, 0, n, np.int64), n, orc.generate_bits(44, 0, 0.95, n), 0, 0, -1)
+    pred = HostArray(BOOL, orc.generate_bits(46, 0, 0.1, n), n, None, 0, 0, 0)
+    a = HostArray(abi.F64, orc.generate_values(2, 42, 0, 0, n, np.float64), n, orc.generate_bits(144, 0, 0.95, n), 0, 0, -1)
+    b = HostArray(abi.F64, orc.generate_values(2, 43, 0, 0, n, np.float64), n, orc.generate_bits(45, 0, 0.95, n), 0, 0, -1)
+    idx = HostArray.from_numpy(abi.U32, np.nonzero(pred.value_array())[0].astype(np.uint32))
+    expect = {"filter": orc.filter(col, pred), "take": orc.take(col, idx), "add": orc.add(a, b)}
+    counts = []
+    for name, e in expect.items():
+        x, v = e.value_array()[: e.length].astype(np.float64), e.valid_mask()
+        x[~v] = 0.0
+        rows = bench.dump_rows(e.length)
+        assert np.array_equal(got[name], x[rows]) and np.array_equal(got[name + "_valid"], v[rows].astype(np.float32)), name
+        counts += [e.length, e.null_count]
+    assert len(got["add"]) == bench.DUMP_ROWS < n and len(got["filter"]) == expect["filter"].length
+    total = orc.sum(expect["take"])
+    assert got["sum"].tolist() == [float(total)]
+    assert got["counts"].tolist() == counts + [expect["take"].length - expect["take"].null_count]
