@@ -12,7 +12,7 @@ import acu
 from acu import _abi as abi
 from acu import BOOL, ArrowError, HostArray
 
-from test_gpu_parity import assert_same, rand_array, rand_bool
+from test_gpu_parity import assert_float_sum, assert_same, rand_array, rand_bool
 
 pytestmark = pytest.mark.gpu
 
@@ -55,9 +55,17 @@ def test_chain_matches_synchronous_calls(gpu, oracle, dtype):
             exp_s = oracle.aggregate(acu.SUM, exp_t)
             if dtype == abi.F64:
                 assert (got_s is None) == (exp_s is None)
-                if exp_s is not None:
-                    # Float64 sum: association order (DESIGN.md section 4); rand_values injects NaN / inf
-                    assert (np.isnan(got_s) and np.isnan(exp_s)) or got_s == pytest.approx(exp_s, rel=1e-9, abs=1e-6)
+                # rand_values injects NaN / inf: NaN exactly when a valid NaN or both infinities were taken
+                sm = gpu.lib.acu_device_sm_count(gpu.h)
+                assert_float_sum(got_s, exp_t.value_array(), exp_t.valid_mask(), dtype, sm, "chain sum " + what)
+                # and the finite rows: the same chain over the column with its specials replaced by 0
+                cv = col.value_array()
+                clean = HostArray(dtype, np.where(np.isfinite(cv), cv, 0.0), n, col.validity, col.validity_offset, 0,
+                                  col.null_count)
+                clean_t = oracle.take(clean, idx)
+                got_c = gpu.chain(clean, pred, idx, a, b, arith_op=op, agg_op=acu.SUM)[3]
+                assert got_c is None or np.isfinite(got_c)
+                assert_float_sum(got_c, clean_t.value_array(), clean_t.valid_mask(), dtype, sm, "chain sum without specials " + what)
             else:
                 assert got_s == exp_s, "chain sum " + what
 

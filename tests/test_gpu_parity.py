@@ -5,10 +5,13 @@ arrow-select/src/filter.rs:1888-1977: random lengths, offsets, null densities vs
 Bar: bit-exact for integer / byte / index / bitmap work, including the bytes written under
 null slots and whether the result carries a NullBuffer at all; floating-point arithmetic is
 compared bit-for-bit except that any NaN matches any NaN (tolerance stated by north_star:
-1 ulp; we hold 0 ulp on non-NaN results). Float `sum` is tolerance-based (order-dependent in
-the reference itself, arrow-arith/src/aggregate.rs:303-313).
+1 ulp; we hold 0 ulp on non-NaN results). Float `sum` is order-dependent in the reference itself
+(arrow-arith/src/aggregate.rs:303-313): it is held to the summation-tree error bound of
+float_sum_bound, and to bit-exactness on order-independent inputs (test_gpu_reduce.py).
 """
 import ctypes as C
+import itertools
+import math
 
 import numpy as np
 import pytest
@@ -54,6 +57,51 @@ def rand_array(rng, dtype, n, null_p, offset=0, small=False):
     return h.slice(offset, n) if offset else h
 
 
+PRECISION = {abi.F32: 24, abi.F64: 53}
+EXACT_KINDS = ("ints", "dyadic", "subnormal", "garbage_under_nulls")
+
+
+def exact_float_array(rng, dtype, n, kind, null_p, offset=0):
+    """A float array whose sum is exact in every association order -> (HostArray, expected sum as a Python float).
+
+    Every value is k·2^e with Σ|k| <= 2^p over the whole buffer (p = 24 for f32, 53 for f64), so every partial sum
+    of any subset, in any order, is representable: the only correct result is Σx itself, bit for bit, and +0.0 when
+    Σx = 0 (the accumulator starts at T::ZERO). kinds: small integers (e = 0), dyadic fractions (e = -20),
+    subnormals (e = the smallest subnormal exponent), and sparse valid integers with NaN / ±inf / huge values in every
+    null slot. `offset` > 0 slices a longer buffer, like rand_array."""
+    npdt = acu.NP_DTYPES[dtype]
+    total = n + offset
+    if kind == "garbage_under_nulls":
+        null_p = 0.9 if null_p is None else max(null_p, 0.9)
+    e = {"ints": 0, "dyadic": -20, "subnormal": -149 if dtype == abi.F32 else -1074, "garbage_under_nulls": 0}[kind]
+    cap = 1000 if dtype == abi.F32 else 1 << 40
+    kmax = max(1, min(cap, (1 << PRECISION[dtype]) // max(total, 1)))
+    k = rng.integers(-kmax, kmax, total, endpoint=True)
+    vals = np.ldexp(k.astype(np.float64), e).astype(npdt)
+    mask = None if null_p is None else rng.random(total) >= null_p
+    if kind == "garbage_under_nulls":
+        junk = np.array([np.nan, -np.nan, np.inf, -np.inf, np.finfo(npdt).max, -np.finfo(npdt).max], dtype=npdt)
+        vals[~mask] = junk[rng.integers(0, len(junk), int((~mask).sum()))]
+    h = HostArray.from_numpy(dtype, vals, mask, bit_offset=int(rng.integers(0, 9)) if mask is not None else 0)
+    if offset:
+        h = h.slice(offset, n)
+    valid = h.valid_mask()
+    kk = k[offset:offset + n][valid]
+    if kk.size == 0:
+        return h, None
+    return h, float(np.array(np.ldexp(float(int(kk.sum())), e), dtype=npdt))
+
+
+def same_float(got, exp, dtype):
+    """Bit-exact float comparison of two Python floats as `dtype` (so +0.0 != -0.0), any NaN matching any NaN."""
+    if got is None or exp is None:
+        return got is None and exp is None
+    if np.isnan(exp):
+        return bool(np.isnan(got))
+    npdt = acu.NP_DTYPES[dtype]
+    return np.array(got, dtype=npdt).tobytes() == np.array(exp, dtype=npdt).tobytes()
+
+
 def rand_bool(rng, n, true_p, null_p, offset=0):
     total = n + offset
     bools = rng.random(total) < true_p
@@ -85,6 +133,59 @@ def assert_same(got, exp, what, float_nan_ok=False, exact_bytes=True):
         if not same_bits(gv[:n], ev[:n]):
             bad = np.nonzero(gv[:n] != ev[:n])[0]
             raise AssertionError(f"{what}: values differ at {bad[:8]}: {gv[bad[:8]]} vs {ev[bad[:8]]}")
+
+
+UNIT_ROUNDOFF = {abi.F32: 2.0 ** -24, abi.F64: 2.0 ** -53}
+
+
+def float_sum_bound(n, dtype, sm_count):
+    """Relative forward-error bound of k_reduce's float sum over an n-row launch: |sum - Σx| <= bound · Σ|x|.
+
+    Recursive summation whose evaluation tree has depth D errs by at most γ_D·Σ|x|, γ_D = D·u / (1 - D·u)
+    (Higham, Accuracy and Stability of Numerical Algorithms, §4.2). D follows the design in reduce.cu's header:
+    sgroups = ⌈n/2048⌉ super-groups, W = ⌈sgroups/8⌉ work blocks of one warp-per-super-group CTA of 8 warps, and a
+    real grid between G_min = min(W, 8·sm_count) (at least one CTA per SM, one wave) and G_max = min(W, 64·sm_count)
+    (at most 8 CTAs per SM, 8 waves). Along any path from a row to the result there are
+      64·⌈sgroups / (8·G_min)⌉   adds into one lane's accumulator (2 rows per 64-row strip, 32 strips per super-group)
+      + 5                        the warp's shuffle tree
+      + 7                        the CTA's fold of its 8 warp partials
+      + ⌈G_max / 32⌉             the last CTA's lane-strided fold of the per-CTA partials
+      + 5                        the final shuffle tree,
+    plus one for the rounding of the reference (math.fsum, correctly rounded in double). Below the grid cap
+    G_min = G_max = W and the bound is exact for the launch; at 70001 rows D = 82 + 1."""
+    if n == 0:
+        return 0.0
+    sgroups = -(-n // 2048)
+    w = -(-sgroups // 8)
+    g_min, g_max = min(w, 8 * sm_count), min(w, 64 * sm_count)
+    depth = 64 * -(-sgroups // (8 * g_min)) + 5 + 7 + -(-g_max // 32) + 5 + 1
+    u = UNIT_ROUNDOFF[dtype]
+    return depth * u / (1 - depth * u)
+
+
+def exact_fsum(x, chunk=1 << 20):
+    """math.fsum over a float array without materialising it as one Python list."""
+    return math.fsum(itertools.chain.from_iterable(x[i:i + chunk].tolist() for i in range(0, len(x), chunk)))
+
+
+def assert_float_sum(got, values, valid, dtype, sm_count, what):
+    """got = the device's float sum of an array of len(values) rows, valid rows marked by `valid`.
+    IEEE outcomes that do not depend on the order are checked exactly (a valid NaN or both infinities: NaN; one
+    infinity: that infinity; no valid row: None); finite sums against math.fsum within float_sum_bound."""
+    x = np.asarray(values)[np.asarray(valid, dtype=bool)].astype(np.float64)
+    if x.size == 0:
+        assert got is None, f"{what}: {got} for a column without valid rows"
+        return
+    assert got is not None, f"{what}: None for {x.size} valid rows"
+    pinf, ninf = bool((x == np.inf).any()), bool((x == -np.inf).any())
+    if np.isnan(x).any() or (pinf and ninf):
+        assert np.isnan(got), f"{what}: {got}, expected NaN"
+    elif pinf or ninf:
+        assert got == (np.inf if pinf else -np.inf), f"{what}: {got}, expected {'+' if pinf else '-'}inf"
+    else:
+        exact = exact_fsum(x)
+        tol = float_sum_bound(len(values), dtype, sm_count) * float(np.abs(x).sum())
+        assert abs(got - exact) <= tol, f"{what}: {got!r} vs fsum {exact!r}: error {abs(got - exact):.3g} > bound {tol:.3g}"
 
 
 def expect_same_error(gpu, oracle, fn):
@@ -607,15 +708,12 @@ def test_aggregate_fuzz(gpu, oracle, dtype):
                     assert np.isnan(g) and np.signbit(g) == np.signbit(e)
                 else:
                     assert g == e, f"{op} dtype={dtype} n={n}: {g} != {e}"
-            if dtype in FLOAT_DTYPES:  # order-dependent: finite inputs, relative tolerance
+            if dtype in FLOAT_DTYPES:  # order-dependent: finite inputs, the summation-tree error bound
                 vals = (rng.random(n) * 2e3 - 1e3).astype(acu.NP_DTYPES[dtype])
                 b = HostArray.from_numpy(dtype, vals, None if null_p is None else rng.random(n) >= null_p)
-                g, e = gpu.sum(b), oracle.sum(b)
-                assert (g is None) == (e is None)
-                if e is not None:
-                    scale = float(np.abs(vals).sum()) + 1.0
-                    tol = (1e-12 if dtype == abi.F64 else 1e-4) * scale  # SURVEY.md §8(a13)
-                    assert abs(g - e) <= tol, f"sum dtype={dtype} n={n}: {g} vs {e}"
+                g = gpu.sum(b)
+                assert (g is None) == (oracle.sum(b) is None)
+                assert_float_sum(g, vals, b.valid_mask(), dtype, gpu.lib.acu_device_sm_count(gpu.h), f"sum dtype={dtype} n={n}")
             else:
                 assert gpu.sum(a) == oracle.sum(a), f"sum dtype={dtype} n={n}"
 

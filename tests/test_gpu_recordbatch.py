@@ -10,7 +10,8 @@ import pytest
 import acu
 from acu import _abi as abi
 from acu import BOOL, HostArray, Utf8Column
-from test_gpu_parity import assert_same, assert_same_bytes, expect_same_error, rand_array, rand_bool, rand_strings
+from test_gpu_parity import (assert_same, assert_same_bytes, exact_float_array, expect_same_error, rand_array, rand_bool,
+                             rand_strings, same_float)
 
 pytestmark = pytest.mark.gpu
 
@@ -116,6 +117,15 @@ def test_aggregate_columns(gpu, oracle):
                     assert np.isnan(got[c]) and np.signbit(got[c]) == np.signbit(exp)
                 else:
                     assert got[c] == exp, f"{op_name} n={n} col {c}: {got[c]} != {exp}"
+        # float sums on order-independent inputs (exact in any association order), in one call with integer sums
+        exact = [exact_float_array(rng, dt, n, kind, null_p, off)
+                 for dt, kind, null_p, off in ((abi.F64, "ints", 0.1, 1), (abi.F32, "dyadic", None, 0),
+                                               (abi.F32, "garbage_under_nulls", 0.9, 3), (abi.F64, "subnormal", None, 2))]
+        use = [h for h, _ in exact] + cols[:2]
+        got = gpu.aggregate_columns([abi.SUM] * len(use), use)
+        for c, (h, e) in enumerate(exact):
+            assert same_float(got[c], e, h.dtype), f"float sum n={n} col {c}: {got[c]!r} != {e!r}"
+        assert got[len(exact):] == [oracle.sum(cols[0]), oracle.sum(cols[1])]
         # mixed ops in one call
         got = gpu.aggregate_columns([abi.SUM, abi.MIN, abi.MAX], cols[:3])
         assert got == [oracle.sum(cols[0]), oracle.min(cols[1]), oracle.max(cols[2])]
